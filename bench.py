@@ -1,7 +1,12 @@
 #!/usr/bin/env python
-"""Benchmark of the AudioGPT generative hot path on B200 (contract: see the task brief).
+"""Benchmark of the AudioGPT generative hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload hifigan|ddim]
+                    [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the timed GPU path returned in its last timed step, rank 0's batch, as float32 .npy
+files: hifigan_wav.npy ([8, 1, 204800] waveforms) and ddim_latent.npy ([4, 4, 10, 78] DDIM end points).  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 BASELINE.json's metric has two halves; one JSON line carries both:
 
@@ -71,6 +76,19 @@ def ddim_config(n_gpus):
             "weights": "seeded random (specs.synth_unet(UNET_TXT2AUDIO, 4040))", "arith": ARITH,
             "parallelism": f"clips sharded x{n_gpus}, no data-path collective",
             "l2_policy": "weights 641 MB fp32 (1.28 GB as fp16 hi/lo images) re-read every forward >> 126 MB L2"}
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every tensor of ``arrays`` as <out_dir>/<name>.npy in float32."""
+    host = {k: v.detach().to("cpu", torch.float32).numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    assert total <= DUMP_MAX_BYTES, f"outputs to dump are {total} bytes, more than {DUMP_MAX_BYTES}"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def load_peaks():
@@ -257,9 +275,10 @@ def run_reference_arm(args):
 
 
 # ------------------------------------------------------------------------------------ GPU arm: DDIM (C4)
-def measure_ddim(dev, rank, n_gpus, chains, peaks, want_cpu, keep=None):
+def measure_ddim(dev, rank, n_gpus, chains, peaks, want_cpu, keep=None, outputs=None):
     """All ranks: DDIM-100 + CFG for DDIM_B clips per rank.  Returns the 'ddim' object (rank 0) or None.
-    ``keep`` (a dict) receives the sampler so that the mixed-dispatch measurement can reuse the 160 M-param engine."""
+    ``keep`` (a dict) receives the sampler so that the mixed-dispatch measurement can reuse the 160 M-param engine;
+    ``outputs`` (a dict) receives the latent of the last timed chain as 'ddim_latent'."""
     import ctypes as C
     import torch.distributed as dist
     from audiogpt_b200 import _lib, parallel, specs
@@ -302,6 +321,8 @@ def measure_ddim(dev, rank, n_gpus, chains, peaks, want_cpu, keep=None):
     barrier()
     ms = e0.elapsed_time(e1)
     launches = _lib.launch_count() - l0
+    if outputs is not None:
+        outputs["ddim_latent"] = z.cpu()
     # e2e: host tensors in, host latent out, through DDIMSampler.sample
     t0 = time.perf_counter()
     for _ in range(chains):
@@ -428,13 +449,16 @@ def run_ours(args):
             dist.barrier()
             dist.destroy_process_group()
 
+    outputs = {}
     if args.workload == "ddim":
         sampler = ClockSampler(local)
         if rank == 0:
             sampler.start()
-        d = measure_ddim(dev, rank, n_gpus, max(1, args.steps), peaks, want_cpu=(n_gpus == 1))
+        d = measure_ddim(dev, rank, n_gpus, args.steps, peaks, want_cpu=(n_gpus == 1), outputs=outputs)
         if rank == 0:
             d["clocks"] = sampler.stop()
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, outputs)
             print(json.dumps(d))
             sys.stdout.flush()
         finish()
@@ -493,13 +517,14 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_device()
+        wav = step_device()
     if gather is not None:
         gather.drain()               # the compute stream waits for every outstanding gather: inside the timed region
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = _lib.launch_count() - l0
+    outputs["hifigan_wav"] = wav.cpu()
     per_rank_ms = None
     if n_gpus > 1:
         allms = [torch.zeros(1, device=dev) for _ in range(n_gpus)]
@@ -586,7 +611,7 @@ def run_ours(args):
     ddim, mixed, keep = None, None, {}
     if not args.no_ddim:
         try:
-            ddim = measure_ddim(dev, rank, n_gpus, args.ddim_chains, peaks, want_cpu=False, keep=keep)
+            ddim = measure_ddim(dev, rank, n_gpus, args.ddim_chains, peaks, want_cpu=False, keep=keep, outputs=outputs)
         except Exception as ex:
             if n_gpus > 1:
                 raise
@@ -635,6 +660,8 @@ def run_ours(args):
             "clocks": clocks, "e2e": e2e, "gpu_launches": int(launches),
             "roofline": roofline, "cpu_baseline": cpu_baseline, "ddim": ddim, "mixed_dispatch": mixed, "extra": extra,
             "waveform_gather": gather_kind, "ms_per_step_by_rank": per_rank_ms}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
     sys.stdout.flush()
     finish()
@@ -732,10 +759,14 @@ def main():
     ap.add_argument("--no-ddim", action="store_true", help="skip the DDIM C4 measurement")
     ap.add_argument("--no-mixed", action="store_true", help="skip the mixed-dispatch (BASELINE configs[4]) measurement")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary DiffSinger / BigVGAN measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, GPU arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
-    if args.workload == "ddim" and args.impl == "ours":
-        args.steps = min(args.steps, 5)
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -313,3 +313,12 @@ def test_bench_reference_arm_contract():
     r1 = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1"],
                         capture_output=True, text=True, timeout=120, env=env, cwd=root)
     assert r1.returncode == 0 and r1.stdout.strip() == ""
+
+
+def test_bench_rejects_bad_arguments(tmp_path):
+    """No timed steps at all, or an output dump from the CPU arm (which times the oracle, not the library)."""
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "out")]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args,
+                           capture_output=True, text=True, timeout=120, cwd=tmp_path)
+        assert r.returncode == 2 and "error:" in r.stderr, (args, r.stderr[-2000:])
+    assert not (tmp_path / "out").exists()

@@ -2,6 +2,10 @@
 CPU oracle, the vocoder wrapper (numpy in / numpy out), and the three generations of the tcgen05
 tap-GEMM kernel against the fp32-FMA kernel on the layer shapes of the BASELINE configs."""
 import ctypes as C
+import json
+import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -13,7 +17,7 @@ from audiogpt_b200.modules.diff.net import DiffNet
 from audiogpt_b200.modules.hifigan.hifigan import HifiGanGenerator
 from audiogpt_b200.utils.hparams import set_hparams_from_dict
 from audiogpt_b200.vocoders.hifigan import HifiGAN, get_vocoder_cls
-from conftest import rel_rmse, rmse
+from conftest import ROOT, rel_rmse, rmse
 
 pytestmark = pytest.mark.gpu
 
@@ -156,3 +160,28 @@ def test_saturating_and_zero_inputs():
     assert rmse(wz, ref) < 2e-6
     big = torch.full((1, 80, 16), 1e6, device="cuda")
     assert torch.isfinite(m(big)).all()
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: the waveforms of the last timed HiFi-GAN step (the same forward on the same seeded
+    mel, run here) and the DDIM end points of the last timed chain; the line reports the --steps it was given."""
+    env = dict(os.environ)
+    env.pop("RANK", None)
+    out = tmp_path / "out"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--ddim-chains", "1",
+                        "--no-mixed", "--no-extra", "--dump-outputs", str(out)],
+                       capture_output=True, text=True, timeout=1200, env=env, cwd=tmp_path)
+    assert r.returncode == 0, r.stderr[-2000:]
+    lines = [l for l in r.stdout.splitlines() if l.strip().startswith("{")]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == 2
+    assert sorted(os.listdir(out)) == ["ddim_latent.npy", "hifigan_wav.npy"]
+    lat = np.load(out / "ddim_latent.npy")
+    assert lat.dtype == np.float32 and lat.shape == (4, 4, 10, 78) and np.isfinite(lat).all()
+    wav = np.load(out / "hifigan_wav.npy")
+    assert wav.dtype == np.float32 and wav.shape == (8, 1, 800 * 256)
+    h = specs.HIFIGAN_V1
+    m = HifiGanGenerator(h)
+    m.load_state_dict(specs.synth_hifigan(h, 1234), strict=True)
+    m = m.eval().to("cuda")
+    ref = m(specs.synth_tensor((8, 80, 800), seed=100, scale=2.0, shift=-4.0).cuda()).cpu()
+    assert rel_rmse(wav, ref) < 1e-6
